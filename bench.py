@@ -3,6 +3,7 @@
 bench.py -- nn-classification throughput (6 kb windows/s) on N B200s, next to the reference's CPU path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config {1,2,3,4,5}] [--batch B] [--impl ours|reference]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -25,6 +26,10 @@ Prints ONE JSON line (rank 0).  BASELINE.json's configs:
              step's windows and D2H of its probabilities inside the timed region)
   roofline : the dominant kernel (tcgen05 Conv1D, conv_t_kernel<false>) against the measured bf16 tensor peak
   cpu_baseline : the oracle's op-for-op restatement of the Keras graph timed on this box's host cores
+
+--dump-outputs DIR (configs 2 and 3) writes the per-window class probabilities of the last timed step, as the caller of the timed
+path receives them (all ranks' windows, gathered), to DIR/probabilities.npy (float32, [N x batch, 3]).  The inputs depend only
+on the arguments, so two builds can be compared output for output.
 
 --impl reference times that CPU restatement (the reference's own implementation is TensorFlow, which cannot be installed
 here -- see DESIGN.md) with all host threads, on bounded 128-window steps.
@@ -314,7 +319,10 @@ def main():
     ap.add_argument("--cpu-windows", type=int, default=512, help="--impl reference: windows per step before the time budget shrinks it")
     ap.add_argument("--no-module", action="store_true", help="skip the module_e2e / config4 extras of the default line")
     ap.add_argument("--module-windows", type=int, default=100_000, help="size of the large module_e2e FASTA (windows)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's probabilities to DIR/probabilities.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.config not in (2, 3)):
+        ap.error("--dump-outputs applies to the timed step loop of --config 2 and 3")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", 0))
@@ -478,6 +486,11 @@ def main():
     total_ms = timed(run_device, use_events=True, tail=exchange)
     launches = per_step * K                                        # our kernels inside the K timed steps
     clocks = sampler.stop() if rank == 0 else None
+    last_probs = None
+    if args.dump_outputs and rank == 0:                            # copied before the stage pass below reuses `probs`
+        m = ((K - 1) % POOL + 1) * B                               # rows of the last API call; its last B rows are the last step
+        src = gathered.view(world, POOL * B, 3) if world > 1 else probs.view(1, POOL * B, 3)
+        last_probs = src[:, m - B:m].reshape(-1, 3).cpu().numpy()
 
     # per-stage CUDA events over K more steps of the same workload (same stream)
     clf.set_option("profile_stages", 1)
@@ -578,6 +591,10 @@ def main():
         if "gather1" in stage_ms:
             line["rooflines_hbm"]["patch_stream_kernel (distinct rows: 4510 x 512 B per window)"] = hbm("gather1", B * 4510 * 512 / 1e9)
         line.update(extras)
+        if last_probs is not None:
+            d = Path(args.dump_outputs)
+            d.mkdir(parents=True, exist_ok=True)
+            np.save(d / "probabilities.npy", last_probs.astype(np.float32))
         if world == 1 and args.cpu_sample > 0:
             # the CPU arm in its own process (no CUDA context to fork): the same code path as `--impl reference`
             r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "1",

@@ -8,6 +8,7 @@ layer, pooling, softmax axes, how the H5 datasets map to layers --, i.e. everyth
 they do not pin is TensorFlow's own fp32 arithmetic.
 
     python tests/golden/make_reference_graph_golden.py     # needs /root/reference; ~2 min -> tests/golden/reference_graph_golden.npz
+    python tests/golden/make_reference_graph_golden.py --rerun     # a second, independent build -> reference_graph_rerun.npz
 
 Stored: token batch (24 windows: 16 of the counter stream incl. N / IUPAC windows + 8 worst-case families), the reference graph's
 probabilities in fp32 and in fp64 arithmetic, with the shipped weights and with synthetic O(1) IGLOO weights (assigned to the
@@ -125,5 +126,21 @@ def main():
     print("wrote", out)
 
 
+def rerun():
+    """Rebuild the reference graph from its source and re-predict three windows of the committed fixture, with the loader's
+    dataset -> variable assignment, into reference_graph_rerun.npz (tests/test_oracle_golden.py compares the fixture with it)."""
+    np.random.seed(0)
+    model_mod, _ = load_reference_model_module()
+    clf = model_mod.create_classifier()
+    clf.load_weights(REF / "data" / "nn_classifier.h5")
+    g = np.load(ROOT / "tests" / "golden" / "reference_graph_golden.npz")
+    pick = np.array([0, 13, 20])
+    p = clf.predict(g["tokens"][pick].astype(np.int64), batch_size=3)
+    report = np.array([f"{a} -> {b} {c} {d}" for a, b, c, d in clf.load_report])
+    out = ROOT / "tests" / "golden" / "reference_graph_rerun.npz"
+    np.savez_compressed(out, pick=pick, shipped=p, load_report=report)
+    print("wrote", out)
+
+
 if __name__ == "__main__":
-    main()
+    rerun() if "--rerun" in sys.argv else main()

@@ -83,11 +83,17 @@ def test_weights_npz_and_shapes(weights_npz):
     assert str(z["__sha256__"]) == "834bcb03aeb1ff484dc7c1f7c00fb951708a91ed03d8a233cd176390930761a1"
 
 
-def test_h5lite_reads_reference_file_if_present(weights_npz):
-    ref = "/root/reference/genomad/data/nn_classifier.h5"
-    import os
-    if not os.path.exists(ref):
-        pytest.skip("reference tree not present on this box")
+def test_h5lite_reads_reference_file_if_present(weights_npz, golden_dir, tmp_path):
+    """The reference's nn_classifier.h5, rebuilt byte for byte from its stored non-payload bytes and the weights' arrays
+    (tests/golden/make_h5_skeleton.py)."""
+    import hashlib
+    import sys
+    sys.path.insert(0, str(golden_dir))
+    import make_h5_skeleton
+    raw = make_h5_skeleton.rebuild(golden_dir / "nn_classifier_h5_skeleton.npz", weights_npz)
+    assert hashlib.sha256(raw).hexdigest() == str(np.load(weights_npz)["__sha256__"])
+    ref = tmp_path / "nn_classifier.h5"
+    ref.write_bytes(raw)
     f = h5lite.H5File(ref)
     z = np.load(weights_npz)
     assert len(f.datasets) == 32

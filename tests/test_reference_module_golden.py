@@ -126,9 +126,10 @@ _EVENTS = (
     ("executing", r"Executinggenomadnn-classification\."),
     ("previous_execution_detected", r"Previousexecutiondetected"),
     ("input_or_parameters_changed", r"Theinputfileortheparameterschanged"),
-    ("mkdir_module", r"Creatingthe[^.]*?toy_nn_classificationdirectory\."),
-    ("mkdir_encoded_sequences", r"Creatingthe[^.]*?toy_encoded_sequencesdirectory\."),
-    ("mkdir_encoded_proviruses", r"Creatingthe[^.]*?toy_encoded_provirusesdirectory\."),
+    # the path may contain dots (e.g. a temporary directory under a user name like first.last): it runs to the first "directory."
+    ("mkdir_module", r"Creatingthe(?:(?!directory\.).)*?/toy_nn_classificationdirectory\."),
+    ("mkdir_encoded_sequences", r"Creatingthe(?:(?!directory\.).)*?/toy_encoded_sequencesdirectory\."),
+    ("mkdir_encoded_proviruses", r"Creatingthe(?:(?!directory\.).)*?/toy_encoded_provirusesdirectory\."),
     ("skip_sequence_encoding", r"toy_encoded_sequenceswasfound\.Skippingsequenceencoding"),
     ("skip_provirus_encoding", r"toy_encoded_proviruseswasfound\.Skippingprovirusencoding"),
     ("encoded_sequences", r"Encodedsequencedatawrittento"),
@@ -246,73 +247,36 @@ def test_module_host_logic_matches_reference_module_run(gold, tmp_path, weights_
     _run_module_and_compare(gold, tmp_path)
 
 
-def test_reference_consumer_accepts_our_outputs(gold, tmp_path, weights_npz, monkeypatch):
+def test_reference_consumer_accepts_our_outputs(gold, golden_dir, tmp_path, weights_npz):
     """Drop-in on the consumer side (INTEGRATION.md level 1): the REFERENCE'S real aggregated-classification module
-    (genomad/modules/aggregated_classification.py, imported by path; build container only) runs on the directory written by
-    genomad_b200's nn-classification module -- its required-file list, the md5 cross-check against our execution-info JSON, the
-    NPZ keys -- and produces what genomad_b200's own aggregated-classification produces from the same files, byte for byte."""
+    (genomad/modules/aggregated_classification.py) ran on a directory written by genomad_b200's nn-classification module -- its
+    required-file list, the md5 cross-check against our execution-info JSON, the NPZ keys -- and what it consumed and produced is
+    stored (tests/golden/reference_consumer/, make_reference_consumer_golden.py).  The same directory written now has the same
+    files and nn-classification NPZs, and genomad_b200's own aggregated-classification produces from those NPZs what the reference
+    produced, byte for byte."""
     import sys
-    if not Path("/root/reference/genomad/modules/aggregated_classification.py").exists():
-        pytest.skip("reference checkout not present")
     from genomad_b200 import aggregated_classification as our_agg
-    sys.path.insert(0, str(Path(__file__).resolve().parent / "golden"))
-    import make_aggregate_golden as G
-    import types
-    w = M.load_npz_weights(weights_npz)
-
-    def oracle_classify(clf, parsed, offsets, info, contig_reduce="gather"):
-        windows = parsed.export_windows(0, parsed.n_windows, np.zeros((max(1, parsed.n_windows), 6000), np.uint8))
-        tok = T.tokenize_windows(windows)
-        p = np.concatenate([M.forward(tok[i:i + 8], w) for i in range(0, len(tok), 8)])
-        return T.segment_mean(p, np.repeat(np.arange(len(offsets) - 1), np.diff(offsets)), len(offsets) - 1)
-    monkeypatch.setattr(nn_classification, "_make_classifier", lambda batch_size, device: object())
-    monkeypatch.setattr(nn_classification, "_classify_parsed", oracle_classify)
-    work = tmp_path / "case"
-    shutil.copytree(gold / "input", work)
-    out = work / "out"
-    out.mkdir()
-    shutil.move(str(work / "toy_find_proviruses"), str(out / "toy_find_proviruses"))
-    fa = work / "toy.fna"
-    nn_classification.main(fa, out, False, 4, False, 2, False, False)
-    # a marker-classification run on the same input (random features / scores; names from our outputs)
-    nn_dir = out / "toy_nn_classification"
-    names = np.load(nn_dir / "toy_nn_classification.npz")["contig_names"]
-    pnames = np.load(nn_dir / "toy_provirus_nn_classification.npz")["provirus_names"]
-    rng = np.random.default_rng(3)
-    mk = out / "toy_marker_classification"
-    mk.mkdir()
-    utils.write_execution_info("marker_classification", fa, {}, mk / "toy_marker_classification.json")
-    np.savez_compressed(mk / "toy_features.npz", contig_names=names, contig_features=rng.random((len(names), 25)).astype(np.float32))
-    np.savez_compressed(mk / "toy_provirus_features.npz", provirus_names=pnames,
-                        provirus_features=rng.random((len(pnames), 25)).astype(np.float32))
-    np.savez_compressed(mk / "toy_marker_classification.npz", contig_names=names, predictions=G._scores(rng, len(names), np.float32))
-    np.savez_compressed(mk / "toy_provirus_marker_classification.npz", provirus_names=pnames,
-                        predictions=G._scores(rng, len(pnames), np.float32))
-    saved = {k: sys.modules.get(k) for k in ("genomad", "genomad._paths", "genomad.utils", "genomad.sequence",
-                                             "genomad.aggregated_classification")}
-    try:
-        agg, ref_utils = G.load_reference_module()
-        ref_utils.metadata = types.SimpleNamespace(version=lambda _name: "reference-from-source")
-        agg.main(fa, out, restart=False, verbose=False)        # sys.exit(1) on any missing file / md5 mismatch
-    finally:
-        for k, v in saved.items():
-            if v is None:
-                sys.modules.pop(k, None)
-            else:
-                sys.modules[k] = v
-    ref_dir = out / "toy_aggregated_classification"
-    ref_files = {p.name: p.read_bytes() for p in ref_dir.iterdir() if p.suffix in (".tsv", ".npz")}
-    assert {"toy_aggregated_classification.tsv", "toy_aggregated_classification.npz",
-            "toy_provirus_aggregated_classification.tsv", "toy_provirus_aggregated_classification.npz"} <= set(ref_files)
-    shutil.rmtree(ref_dir)
-    (out / "toy_aggregated_classification.log").unlink()
+    sys.path.insert(0, str(golden_dir))
+    import make_reference_consumer_golden as G
+    ref = golden_dir / "reference_consumer"
+    fa, out = G.build_case(gold, tmp_path / "case", weights_npz)
+    files = sorted(str(p.relative_to(out)) for p in out.rglob("*") if p.is_file())
+    assert files == json.loads((ref / "files.json").read_text())
+    for npz, key in (("toy_nn_classification.npz", "contig_names"), ("toy_provirus_nn_classification.npz", "provirus_names")):
+        z, r = np.load(out / "toy_nn_classification" / npz), np.load(ref / "consumed" / npz)
+        assert sorted(z.files) == sorted(r.files) == sorted([key, "predictions"])
+        assert z[key].tolist() == r[key].tolist() and z[key].dtype == r[key].dtype
+        assert z["predictions"].dtype == r["predictions"].dtype and np.abs(z["predictions"] - r["predictions"]).max() <= 1e-6
+        shutil.copy(ref / "consumed" / npz, out / "toy_nn_classification" / npz)     # the reference's exact inputs
     our_agg.main(fa, out, restart=False, verbose=False)
-    for name, blob in ref_files.items():
+    expected = sorted(p.name for p in (ref / "expected").iterdir())
+    assert expected == ["toy_aggregated_classification.npz", "toy_aggregated_classification.tsv",
+                        "toy_provirus_aggregated_classification.npz", "toy_provirus_aggregated_classification.tsv"]
+    for name in expected:
         if name.endswith(".tsv"):
-            assert (out / "toy_aggregated_classification" / name).read_bytes() == blob, name
+            assert (out / "toy_aggregated_classification" / name).read_bytes() == (ref / "expected" / name).read_bytes(), name
         else:
-            import io
-            z, r = np.load(out / "toy_aggregated_classification" / name), np.load(io.BytesIO(blob))
+            z, r = np.load(out / "toy_aggregated_classification" / name), np.load(ref / "expected" / name)
             assert sorted(z.files) == sorted(r.files)
             for k in z.files:
                 assert z[k].dtype == r[k].dtype and np.array_equal(z[k], r[k]), (name, k)
